@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                 # config 2 (default): the BASELINE metric, our arm
     python bench.py --config {2,3,4,5} ...                         # 3: YOLO-NAS-M train, 4: ResNet-50 train, 5: POSE-L predict()
     python bench.py --impl reference [--config C] --gpus N ...     # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR                         # also write what the last timed step computed, DIR/<name>.npy
 
   config 2  YOLO-NAS-S  640x640 train step, 32 images / GPU (fwd + PPYoloELoss/TAL + bwd + AdamW + EMA)      [BASELINE metric]
   config 3  YOLO-NAS-M  640x640 train step, 16 images / GPU (same step; the weak-scaling sweep config)
@@ -150,6 +151,38 @@ class ClockSampler:
             self.proc = None
 
 
+DUMP_SAMPLE = 1 << 20  # elements kept of an output larger than this (a fixed, seeded sample)
+
+
+def param_sample(step):
+    """The trained parameters (and their EMA) after the step, as a seeded sample taken in parameter-NAME order: two builds whose flat
+    parameter layout differs still sample the same elements."""
+    import torch
+
+    f = step.flat
+    pos = torch.cat([torch.arange(off, off + k) for _, (off, k) in sorted(f.offsets.items())])
+    if pos.numel() > DUMP_SAMPLE:
+        pos = pos[torch.randperm(pos.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values]
+    pos = pos.to(f.params.device)
+    out = {"params_sample": f.params[pos]}
+    if step.ema_on:
+        out["ema_params_sample"] = step.ema_params[pos]
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor} as out_dir/<name>.npy: float64 stays float64, other floating types become float32, integers float64
+    (exact up to 2**53)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu()
+        a = a.double() if a.dtype == torch.float64 or not a.is_floating_point() else a.float()
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -289,7 +322,7 @@ def run_reference(args, cfg):
         return
     cores = os.cpu_count() or 1
     threads = pick_cpu_threads(cores)
-    ips, sec, n, sample, cold = cpu_sample_rate(cfg, threads, max_steps=max(1, min(args.steps, 3)) + 1, budget_s=120.0)
+    ips, sec, n, sample, cold = cpu_sample_rate(cfg, threads, max_steps=args.steps + 1, budget_s=float("inf"))  # one cold step + --steps timed
     what = {"train_det": "train step", "train_cls": "train step", "predict_pose": "predict() batch"}[cfg["kind"]]
     line = {
         "impl": "reference", "metric": cfg["metric"], "value": ips, "unit": "images/sec", "n_gpus": args.gpus, "steps": n, "warmup": cold,
@@ -418,10 +451,10 @@ def run_train(args, cfg):
         if prof_range:
             torch.cuda.profiler.start()
         e0.record()
-        loss = None
+        out = None
         for i in range(args.steps):
             step.set_hyper_params(lr_at(i), ema_decay)
-            loss, _ = step.run(dev_x[i % nbuf], dev_t[i % nbuf])
+            out = step.run(dev_x[i % nbuf], dev_t[i % nbuf])
         e1.record()
         barrier()
         if prof_range:
@@ -432,9 +465,14 @@ def run_train(args, cfg):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms, clocks, loss
+        return ms, clocks, out
 
-    ms, clocks, loss = timed_region()
+    ms, clocks, (loss, items) = timed_region()
+    # what the last timed step computed, copied before anything else runs (a captured graph's outputs are rewritten by every replay).
+    # A re-measured region below continues training, so the outputs are those of the first region: independent of the clocks.
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = {"loss": loss.clone(), "loss_items": items.clone(), **param_sample(step)}
     # a thermally / hardware-throttled region, or clocks pinned far below max without a reason, is measured once more (every
     # rank follows rank 0's verdict: the region contains collectives)
     bad = {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"} & set(clocks.get("reasons", []))
@@ -444,7 +482,7 @@ def run_train(args, cfg):
         dist.broadcast(redo, src=0)
     if int(redo) == 1 and not prof_range:
         first = clocks
-        ms, clocks, loss = timed_region()
+        ms, clocks, (loss, _) = timed_region()
         clocks["remeasured_after"] = {"reasons": first.get("reasons"), "sm_mhz": first.get("sm_mhz")}
     sampler.stop()
     final_loss = float(loss)
@@ -513,6 +551,8 @@ def run_train(args, cfg):
 
     if rank != 0:
         return
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     cpu = None
     if not args.skip_cpu_baseline and world == 1:
         cpu = cpu_baseline(cfg)
@@ -662,6 +702,8 @@ def run_predict(args, cfg):
     K.PROFILE_ON[0] = False
     if rank != 0:
         return
+    if args.dump_outputs:  # the last timed step's device-resident result (forward_batched)
+        dump_outputs(args.dump_outputs, dict(zip(("rows", "poses", "anchor_index", "count"), out)))
     roof = conv_roofline(K.PROFILE, n_prof, cfg, batch, ms / args.steps, args.config)
     per = {}
     for name, a, b, _tag in K.PROFILE:
@@ -705,7 +747,12 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: the configuration's)")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)

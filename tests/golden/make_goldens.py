@@ -695,6 +695,27 @@ def golden_param_groups():
     torch.save(out, os.path.join(HERE, "param_groups.pt"))
 
 
+def golden_collate_decoding():
+    """DetectionCollateFN / YoloNASPoseCollateFN (collate_fn/detection_collate_fn.py, yolo_nas_pose_collate_fn.py) and the export
+    graph's YoloNASDecodingModule / YoloNASPoseDecodingModule (yolo_nas_variants.py:53-72, yolo_nas_pose_variants.py:54-90) on the
+    seeded inputs of tests/test_host_logic.py."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_host_logic as T
+    from super_gradients.training.datasets.pose_estimation_datasets.yolo_nas_pose_collate_fn import YoloNASPoseCollateFN
+    from super_gradients.training.models.detection_models.yolo_nas.yolo_nas_variants import YoloNASDecodingModule
+    from super_gradients.training.models.pose_estimation_models.yolo_nas_pose.yolo_nas_pose_variants import YoloNASPoseDecodingModule
+    from super_gradients.training.utils.collate_fn.detection_collate_fn import DetectionCollateFN
+
+    det_images, det_targets = DetectionCollateFN()(T._collate_samples(0))
+    pose_images, pose_targets, _ = YoloNASPoseCollateFN()(T._pose_samples(1))
+    boxes, scores, conf, coords, js = T._decoding_inputs(0)
+    out = dict(
+        det_images=det_images, det_targets=det_targets, pose_images=pose_images, pose_targets=pose_targets,
+        det_decoded=YoloNASDecodingModule(100)(((boxes, scores), None)), pose_decoded=YoloNASPoseDecodingModule(64)(((boxes, conf, coords, js), None)),
+    )  # fmt: skip
+    torch.save(out, os.path.join(HERE, "collate_decoding.pt"))
+
+
 def golden_tiny_yolo_nas():
     from super_gradients.training.losses.ppyolo_loss import PPYoloELoss
     from super_gradients.training.models.detection_models.yolo_nas.yolo_nas_variants import YoloNAS
@@ -899,7 +920,7 @@ def golden_droppath():
 
 if __name__ == "__main__":
     ref_shim.install()
-    which = sys.argv[1:] or ["qarepvgg", "conv_blocks", "loss", "atss", "nms", "yolox_nms", "processing", "detection_metrics", "lr_schedules", "param_groups", "pose_nms", "pose", "tiny_yolo_nas", "tiny_yolo_nas_pose", "tiny_yolo_nas_pose_train", "state_keys", "resnet_cifar_train", "other_configs", "port_fidelity"]
+    which = sys.argv[1:] or ["qarepvgg", "conv_blocks", "loss", "atss", "nms", "yolox_nms", "processing", "detection_metrics", "lr_schedules", "param_groups", "collate_decoding", "pose_nms", "pose", "tiny_yolo_nas", "tiny_yolo_nas_pose", "tiny_yolo_nas_pose_train", "state_keys", "resnet_cifar_train", "other_configs", "port_fidelity"]
     for w in which:
         print("generating", w, flush=True)
         globals()["golden_" + w]()

@@ -7,7 +7,10 @@ addresses: without a GPU the entry point either rejects the descriptor (SGB_E_IN
 library cannot serve, which would be the first thing to fail on hardware) or gets as far as the first CUDA call and returns
 SGB_E_CUDA.  No kernel runs, nothing is read through the pointers on the host."""
 import collections
+import functools
 import os
+import re
+import subprocess
 import sys
 
 import pytest
@@ -25,6 +28,23 @@ from super_gradients_b200 import lib as L  # noqa: E402
 # list: nothing to validate through the C entry point
 TABLES = {"weight_prepare_batch", "run_weight_prepare_batch", "wgrad_to_oihw_batch_table", "run_wgrad_to_oihw_batch", "qarep_alpha_finish_table", "run_qarep_alpha_finish"}
 REAL = {name: getattr(K, name) for name in list(cpu_backend._SUBSET) + list(cpu_backend._TRAINING) if hasattr(K, name) and name not in TABLES}
+
+
+def without_gpu(test):
+    """The tests below pass host tensors' addresses to the real entry points and rely on there being no CUDA device, so that a valid
+    call stops at its first CUDA call (SGB_E_CUDA).  Where a GPU is visible such a call would launch kernels on host addresses;
+    there the test runs in a child pytest process that sees no GPU (CUDA_VISIBLE_DEVICES empty) and must pass in it."""
+
+    @functools.wraps(test)
+    def run(*args, **kwargs):
+        if not torch.cuda.is_available():
+            return test(*args, **kwargs)
+        node = os.environ["PYTEST_CURRENT_TEST"].rsplit(" ", 1)[0]
+        out = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", node], cwd=os.path.dirname(HERE),
+                             env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=850)  # fmt: skip
+        assert out.returncode == 0 and re.search(r"\b1 passed\b", out.stdout), out.stdout[-3000:] + out.stderr[-2000:]
+
+    return run
 
 
 @pytest.fixture
@@ -84,6 +104,7 @@ def _median_log_ratio(mine, ref):
 
 
 @pytest.mark.parametrize("name", ["yolo_nas_m", "yolo_nas_l"])
+@without_gpu
 def test_yolo_nas_m_l_train_step_shapes_are_served(validating_backend, name):
     """One AdamW + EMA train step of YOLO-NAS-M / -L at 128 x 128.  For M (config 3) the raw head outputs, the loss components and
     the per-parameter gradient norms are compared with the unmodified reference's (same seeded initialisation)."""
@@ -114,6 +135,7 @@ def test_yolo_nas_m_l_train_step_shapes_are_served(validating_backend, name):
         assert l2rel(eb, g["eval_boxes"]) < 0.03 and l2rel(es, g["eval_scores"]) < 0.03
 
 
+@without_gpu
 def test_resnet50_train_step_shapes_are_served(validating_backend):
     """Config 4's model: train-mode logits, cross-entropy, gradients and eval-mode logits against the reference's."""
     from super_gradients_b200.training import models
@@ -140,6 +162,7 @@ def test_resnet50_train_step_shapes_are_served(validating_backend):
         assert l2rel(m(g["x"].float()), g["eval_logits"]) < 0.08
 
 
+@without_gpu
 def test_yolo_nas_pose_l_predict_shapes_are_served(validating_backend):
     """Config 5's model: decoded eval outputs against the reference's, then predict() (NMS path) for the call coverage."""
     from super_gradients_b200.training import models
@@ -158,6 +181,7 @@ def test_yolo_nas_pose_l_predict_shapes_are_served(validating_backend):
     assert l2rel(scores, g["scores"]) < 0.05 and l2rel(joint_scores, g["joint_scores"]) < 0.05
 
 
+@without_gpu
 def test_the_validation_hook_sees_rejections(validating_backend):
     """Negative control: a descriptor the library must refuse is reported, an acceptable one is not."""
     import ctypes
@@ -174,6 +198,7 @@ def test_the_validation_hook_sees_rejections(validating_backend):
     assert len(rejected) == 1 and rejected[0][1] == -1
 
 
+@without_gpu
 def test_new_entry_points_validate_their_descriptors(monkeypatch):
     """sgb_atss_assign / sgb_detection_matching / sgb_focal_cls_fwd_bwd through the product wrappers with host tensors: a valid call
     reaches the first CUDA call (SGB_E_CUDA here), an invalid one is refused with SGB_E_INVALID and the reason."""
@@ -205,6 +230,7 @@ def test_new_entry_points_validate_their_descriptors(monkeypatch):
     assert "code -3" in code(focal)
 
 
+@without_gpu
 def test_replaced_input_channels_are_served(validating_backend):
     """models.get(..., num_input_channels=N): 1-channel ResNet-18 and 4-channel YOLO-NAS-S forward + backward run, and the first
     layers' (channel-padded) shapes pass the C-ABI validation."""

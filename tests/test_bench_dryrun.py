@@ -48,3 +48,22 @@ def test_bench_remeasures_a_throttled_region_on_every_rank():
     assert out.stderr.count("finished") == 2
     line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][0])
     assert line["clocks"]["reasons"] == [] and line["clocks"]["remeasured_after"]["reasons"] == ["hw_slowdown"]
+
+
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs writes the last timed step's loss, its items and a sample of the trained parameters and of their EMA as float32 /
+    float64 .npy files within 64 MB.  The same arguments give the same inputs and the same arrays; another --steps trains further."""
+    import numpy as np
+
+    runs = {"a": (), "b": (), "c": ("--steps", "3")}
+    for port, (name, flags) in zip((29545, 29546, 29547), runs.items()):
+        out = _run(1, port, "--dump-outputs", str(tmp_path / name), *flags)
+        assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-4000:]
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["ema_params_sample.npy", "loss.npy", "loss_items.npy", "params_sample.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 << 20
+    for n in names:
+        a, b, c = (np.load(tmp_path / r / n) for r in runs)
+        assert a.dtype in (np.float32, np.float64) and a.size and np.isfinite(a).all(), n
+        assert np.array_equal(a, b), n
+    assert not np.array_equal(np.load(tmp_path / "a" / "params_sample.npy"), np.load(tmp_path / "c" / "params_sample.npy"))

@@ -270,6 +270,18 @@ def test_replace_input_channels_and_checkpoint_num_classes(tmp_path):
     assert {k: tuple(v.shape) for k, v in y.state_dict().items() if "stem" in k and "3x3.conv.weight" in k}.popitem()[1][1] == 4
 
 
+def _collate_samples(seed):
+    gen = np.random.RandomState(seed)
+    return [(gen.rand(16, 24, 3).astype(np.float32), gen.rand(n, 5).astype(np.float32) * 10) for n in (3, 0, 2)]
+
+
+def _decoding_inputs(seed):
+    """Head outputs of 3 images x 400 anchors: boxes, 80 class scores, and the pose head's confidence, 17 joints' coordinates and scores."""
+    gen = torch.Generator().manual_seed(seed)
+    boxes, scores = torch.rand(3, 400, 4, generator=gen), torch.rand(3, 400, 80, generator=gen)
+    return boxes, scores, torch.rand(3, 400, 1, generator=gen), torch.rand(3, 400, 17, 2, generator=gen), torch.rand(3, 400, 17, generator=gen)
+
+
 def _pose_samples(seed):
     import types
 
@@ -281,18 +293,17 @@ def _pose_samples(seed):
     return samples
 
 
-def test_collate_functions_produce_the_reference_target_formats():
+def test_collate_functions_produce_the_reference_target_formats(golden):
     """DetectionCollateFN (detection_collate_fn.py:10-49) and YoloNASPoseCollateFN / flat_collate_tensors_with_batch_index
     (yolo_nas_pose_collate_fn.py:14-123): the producers of the flat target tensors rows L1 / L7 consume -- equal to the reference's
-    outputs when /root/reference is present, and accepted by the product's target padding either way."""
+    outputs (tests/golden/collate_decoding.pt) and accepted by the product's target padding."""
     from super_gradients_b200.common.registry import COLLATE_FUNCTIONS
     from super_gradients_b200.training.datasets.pose_estimation_datasets import YoloNASPoseCollateFN, flat_collate_tensors_with_batch_index, undo_flat_collate_tensors_with_batch_index
     from super_gradients_b200.training.losses.ppyolo_loss import pad_targets_host
     from super_gradients_b200.training.losses.yolo_nas_pose_loss import pad_pose_targets_host
     from super_gradients_b200.training.utils.collate_fn import DatasetItemsException, DetectionCollateFN
 
-    gen = np.random.RandomState(0)
-    data = [(gen.rand(16, 24, 3).astype(np.float32), gen.rand(n, 5).astype(np.float32) * 10) for n in (3, 0, 2)]
+    data = _collate_samples(0)
     images, targets = DetectionCollateFN()(data)
     assert images.shape == (3, 3, 16, 24) and images.dtype == torch.float32 and targets.shape == (5, 6) and targets[:, 0].tolist() == [0, 0, 0, 2, 2]
     assert torch.equal(targets[3:, 1:], torch.from_numpy(data[2][1])) and COLLATE_FUNCTIONS["DetectionCollateFN"] is DetectionCollateFN
@@ -315,33 +326,19 @@ def test_collate_functions_produce_the_reference_target_formats():
     padded = pad_pose_targets_host((b.float(), j.float(), c), 3, 4)
     assert padded[-1].sum(1).tolist() == [2, 0, 3]
 
-    # against the reference itself, in a child process (the import shim installs module stubs that must not leak into this one)
-    if not os.path.isdir("/root/reference/src/super_gradients"):
-        return
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    child = (
-        "import sys, torch, numpy as np; sys.path[:0] = [%r, %r]\n"
-        "import test_host_logic as T\n"
-        "from oracle import ref_shim; ref_shim.install()\n"
-        "from super_gradients.training.datasets.pose_estimation_datasets.yolo_nas_pose_collate_fn import YoloNASPoseCollateFN as RefPose\n"
-        "from super_gradients.training.utils.collate_fn.detection_collate_fn import DetectionCollateFN as RefDet\n"
-        "from super_gradients_b200.training.datasets.pose_estimation_datasets import YoloNASPoseCollateFN\n"
-        "from super_gradients_b200.training.utils.collate_fn import DetectionCollateFN\n"
-        "gen = np.random.RandomState(0)\n"
-        "data = [(gen.rand(16, 24, 3).astype(np.float32), gen.rand(n, 5).astype(np.float32) * 10) for n in (3, 0, 2)]\n"
-        "(ri, rt), (pi, pt) = RefDet()(data), DetectionCollateFN()(data)\n"
-        "assert torch.equal(ri, pi) and torch.equal(rt, pt) and rt.dtype == pt.dtype\n"
-        "ra, (rb, rj, rc), _ = RefPose()(T._pose_samples(1)); pa, (pb, pj, pc), _ = YoloNASPoseCollateFN()(T._pose_samples(1))\n"
-        "assert torch.equal(ra, pa) and torch.equal(rb, pb) and torch.equal(rj, pj) and torch.equal(rc, pc) and rb.dtype == pb.dtype and rc.dtype == pc.dtype\n"
-        "print('same as the reference')\n"
-    ) % (root, os.path.join(root, "tests"))
-    out = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and "same as the reference" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
+    # against the reference's outputs on the same inputs
+    g = golden("collate_decoding")
+    pi, pt = DetectionCollateFN()(_collate_samples(0))
+    assert torch.equal(g["det_images"], pi) and torch.equal(g["det_targets"], pt) and g["det_targets"].dtype == pt.dtype
+    pa, (pb, pj, pc), _ = YoloNASPoseCollateFN()(_pose_samples(1))
+    ra, (rb, rj, rc) = g["pose_images"], g["pose_targets"]
+    assert torch.equal(ra, pa) and torch.equal(rb, pb) and torch.equal(rj, pj) and torch.equal(rc, pc) and rb.dtype == pb.dtype and rc.dtype == pc.dtype
 
 
-def test_export_decoding_modules_match_the_reference():
+def test_export_decoding_modules_match_the_reference(golden):
     """Row N4: YoloNASDecodingModule (yolo_nas_variants.py:53-72) and YoloNASPoseDecodingModule (yolo_nas_pose_variants.py:54-90),
-    the pre-NMS top-k of the export graph, against the reference's modules on the same random head outputs (child process)."""
+    the pre-NMS top-k of the export graph, against the reference's modules' outputs on the same random head outputs
+    (tests/golden/collate_decoding.pt)."""
     from super_gradients_b200.training.models.detection_models.yolo_nas import YoloNASDecodingModule
     from super_gradients_b200.training.models.pose_estimation_models.yolo_nas_pose.yolo_nas_pose_variants import YoloNASPoseDecodingModule
 
@@ -354,25 +351,12 @@ def test_export_decoding_modules_match_the_reference():
     assert pb.shape == (2, 8, 4) and pc.shape == (2, 8, 1) and pj.shape == (2, 8, 5, 3) and (pc[:, :, 0].diff(dim=1) <= 0).all()
     k = int(conf[0, :, 0].argmax())
     assert torch.equal(pb[0, 0], boxes[0, k]) and torch.equal(pj[0, 0, :, :2], coords[0, k]) and torch.equal(pj[0, 0, :, 2], js[0, k])
-    if not os.path.isdir("/root/reference/src/super_gradients"):
-        return
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    child = (
-        "import sys, torch; sys.path[:0] = [%r]\n"
-        "from oracle import ref_shim; ref_shim.install()\n"
-        "from super_gradients.training.models.detection_models.yolo_nas.yolo_nas_variants import YoloNASDecodingModule as RD\n"
-        "from super_gradients.training.models.pose_estimation_models.yolo_nas_pose.yolo_nas_pose_variants import YoloNASPoseDecodingModule as RP\n"
-        "from super_gradients_b200.training.models.detection_models.yolo_nas import YoloNASDecodingModule as PD\n"
-        "from super_gradients_b200.training.models.pose_estimation_models.yolo_nas_pose.yolo_nas_pose_variants import YoloNASPoseDecodingModule as PP\n"
-        "gen = torch.Generator().manual_seed(0)\n"
-        "boxes, scores = torch.rand(3, 400, 4, generator=gen), torch.rand(3, 400, 80, generator=gen)\n"
-        "for a, b in zip(RD(100)(((boxes, scores), None)), PD(100)(((boxes, scores), None))): assert torch.equal(a, b)\n"
-        "conf, coords, js = torch.rand(3, 400, 1, generator=gen), torch.rand(3, 400, 17, 2, generator=gen), torch.rand(3, 400, 17, generator=gen)\n"
-        "for a, b in zip(RP(64)(((boxes, conf, coords, js), None)), PP(64)(((boxes, conf, coords, js), None))): assert torch.equal(a, b)\n"
-        "print('same as the reference')\n"
-    ) % (root,)
-    out = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and "same as the reference" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
+    g = golden("collate_decoding")
+    boxes, scores, conf, coords, js = _decoding_inputs(0)
+    det, pose = YoloNASDecodingModule(100)(((boxes, scores), None)), YoloNASPoseDecodingModule(64)(((boxes, conf, coords, js), None))
+    assert len(det) == len(g["det_decoded"]) and len(pose) == len(g["pose_decoded"])
+    for a, b in zip((*g["det_decoded"], *g["pose_decoded"]), (*det, *pose)):
+        assert torch.equal(a, b)
 
 
 def test_flat_state_adjacency_requests_and_checkpoint_remap(tmp_path):
